@@ -2,9 +2,11 @@
 """bench.py -- SDXL 50-step latency (ms/image) of the B200-native patch-parallel UNet path.
 
     python bench.py --gpus 1 --steps 5 --warmup 3                       # ours, one GPU
+    python bench.py ... --dump-outputs DIR                              # also write the last timed image's latents
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...                                # the reference's CPU path (oracle port), host cores
     python bench.py --impl reference-gpu ...                            # extra: the UNMODIFIED reference on the same GPUs
+                                                                        # (needs it installed under baseline/_ref: DESIGN.md 6)
 
 A "step" of our arm is one full image: 50 denoising steps (CFG pair per step) of the SDXL UNet at --resolution (default
 1024x1024 = BASELINE.json configs[1]'s workload; strong scaling: the same image at every N), Euler scheduler, 4 warm-up
@@ -56,7 +58,21 @@ def parse():
     ap.add_argument("--no-hires", action="store_true", help="skip the 3840x3840 block")
     ap.add_argument("--hires-resolution", type=int, default=3840)
     ap.add_argument("--cpu-budget-s", type=float, default=200.0, help="wall budget of the CPU reference arm")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the latents the last timed image returned to DIR/images.npy (float32), to compare two builds")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs is not None:
+        if a.impl != "ours":
+            ap.error("--dump-outputs applies to --impl ours")
+        try:                                                    # fail before the timed run, not after it
+            os.makedirs(a.dump_outputs, exist_ok=True)
+        except OSError as e:
+            ap.error(f"--dump-outputs: {e}")
+        if not os.access(a.dump_outputs, os.W_OK):
+            ap.error(f"--dump-outputs: {a.dump_outputs} is not writable")
+    return a
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -239,7 +255,9 @@ def run_reference_gpu(a):
     the denoising loop is the same latent-space stand-in our arm uses.  Reported as an extra arm; never the `reference` slot."""
     ref_dir = os.path.join(ROOT, "baseline", "_ref")
     if not os.path.isdir(os.path.join(ref_dir, "distrifuser")):
-        print_json(json.dumps({"impl": "reference-gpu", "unavailable": "baseline/_ref/distrifuser is not installed"}))
+        print_json(json.dumps({"impl": "reference-gpu", "unavailable": "baseline/_ref/distrifuser is not installed (a clean checkout does "
+                                                                        "not have it: pip install --no-deps --target baseline/_ref <a distrifuser "
+                                                                        "source tree>)"}))
         return
     sys.path.insert(0, os.path.join(ROOT, "oracle", "diffusers_stub"))
     sys.path.insert(0, ref_dir)
@@ -527,6 +545,21 @@ def step_times(pipe, cfg, reps=8):
     return out
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """Writes each tensor as out_dir/<name>.npy in float32.  The bench inputs and weights come from fixed seeds, so two
+    builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    host = {name: t.detach().float().cpu().numpy() for name, t in arrays.items()}
+    total = sum(x.nbytes for x in host.values())
+    if total > DUMP_MAX_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_MAX_BYTES}-byte limit")
+    for name, x in host.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), x)
+
+
 def run_ours(a):
     import torch
     from torch import distributed as dist
@@ -548,6 +581,7 @@ def run_ours(a):
                 io_["out_h"].copy_(r.images, non_blocking=True)
             else:
                 r = pipe_(prompt_embeds=io_["embeds_d"], pooled_prompt_embeds=io_["pooled_d"], latents=io_["lat_d"], **kw)
+            io_["images"] = r.images                        # a fresh tensor per image: later images do not overwrite it
             return r
         return image
     image = make_image(pipe, io)
@@ -579,6 +613,7 @@ def run_ours(a):
     n0 = _lib.LAUNCHES["total"]
     total_ms = timed(image, False, a.steps)
     launches = _lib.LAUNCHES["total"] - n0
+    timed_images = io["images"]                             # what the last timed image returned (written by --dump-outputs)
     e2e_ms = timed(image, True, a.steps)
     clocks = sampler.stop() if rank == 0 else None
     ms_image = total_ms / a.steps
@@ -675,6 +710,8 @@ def run_ours(a):
                 "e2e": {"value": ms_image_e2e, "unit": "ms/image", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": io["out_h"].numel() * 4},
                 "gpu_launches": launches, "clocks": clocks}
         print_json(json.dumps(line))
+        if a.dump_outputs is not None:                        # after the line: a failed dump does not lose the measurement
+            dump_outputs(a.dump_outputs, {"images": timed_images})
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()

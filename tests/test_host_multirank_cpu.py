@@ -50,7 +50,8 @@ def _worker(rank, world, port, cfg_on, split, outdir):
 
 
 @pytest.mark.parametrize("world,cfg_on,split", [(2, True, True), (2, True, False), (4, True, True), (4, False, True)])
-def test_config_and_arena_layout_multirank(world, cfg_on, split):
+def test_config_and_arena_layout_multirank(world, cfg_on, split, monkeypatch):
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")      # the spawned ranks take the host path on GPU machines too
     with tempfile.TemporaryDirectory() as d:
         mp.spawn(_worker, args=(world, free_port(), cfg_on, split, d), nprocs=world, join=True)
         assert len(os.listdir(d)) == world
