@@ -13,12 +13,14 @@ NBANKS = 3
 MAX_WORLD = 8
 IPC_HANDLE_BYTES = 64
 TENSORMAP_BYTES = 128
+AR_RING = 2          # DF_AR_RING: depth of the all-reduce slot ring (tensor parallelism)
 
 EXPORTS = (
     "df_last_error", "df_version", "df_device_sm_count", "df_symm_alloc", "df_symm_open", "df_symm_close",
     "df_symm_free", "df_step_begin", "df_slot_publish", "df_slot_wait", "df_groupnorm_scratch_bytes",
     "df_groupnorm_fwd", "df_groupnorm_halo_fwd", "df_halo_push", "df_halo_assemble", "df_attn_make_kvmaps", "df_attn_workspace_bytes", "df_attn_fwd",
     "df_output_gather", "df_geglu", "df_add_layernorm", "df_bias_residual_add", "df_linear_supported", "df_linear_geglu_block", "df_linear_fwd",
+    "df_allreduce_fwd",
 )
 
 
@@ -70,6 +72,7 @@ def lib():
         L.df_linear_geglu_block.argtypes = [i64, i32, i32]
         L.df_linear_fwd.argtypes = [DfComm, vp, vp, vp, vp, vp, i64, i32, i32, i64, i64, i64, i64, i32, i32, i32, i32, i32, u32, u64,
                                     u64, i32, vp]
+        L.df_allreduce_fwd.argtypes = [DfComm, vp, vp, i64, i32, vp, vp, u32, i32, i32, u64, u64, u64, i32, vp]
         L.df_output_gather.argtypes = [DfComm, vp, vp, i32, i32, i32, i32, i32, i32, i32, i32, i32, u64, vp]
         for name in EXPORTS:
             getattr(L, name)  # AttributeError if the header and the library disagree
@@ -80,7 +83,7 @@ def lib():
 # kernels launched per C-ABI call (bench.py reports the count of OUR launches inside the timed region)
 KERNELS_PER_CALL = {"df_groupnorm_fwd": 1, "df_groupnorm_halo_fwd": 1, "df_attn_fwd": 1, "df_halo_push": 1, "df_halo_assemble": 1,
                     "df_slot_publish": 1, "df_slot_wait": 1, "df_step_begin": 1, "df_output_gather": 2, "df_geglu": 1, "df_add_layernorm": 1, "df_bias_residual_add": 1,
-                    "df_linear_fwd": 1}
+                    "df_linear_fwd": 1, "df_allreduce_fwd": 1}
 LAUNCHES = {"total": 0}
 PROFILE = None   # bench.py sets this to a list; kernels then bracket their launch with CUDA events on the launching stream
 

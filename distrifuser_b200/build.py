@@ -10,7 +10,7 @@ import subprocess
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libdistrifuser_b200.so")
-SOURCES = ("comm.cu", "groupnorm.cu", "halo.cu", "attention.cu", "elementwise.cu", "linear.cu")
+SOURCES = ("comm.cu", "groupnorm.cu", "halo.cu", "attention.cu", "elementwise.cu", "linear.cu", "allreduce.cu")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
          "-Xcompiler", "-fPIC", "-shared"]
 

@@ -62,6 +62,19 @@ class DistriUNetPP(BaseModel):  # for Patch Parallelism
         model.to(memory_format=torch.channels_last)
         super().__init__(model, distri_config)
 
+    def _graph_index(self) -> int:
+        cfg = self.distri_config
+        if self.counter <= cfg.warmup_steps:                         # distri_sdxl_unet_pp.py:108-113
+            return 0
+        return 1 if self.counter == cfg.warmup_steps + 1 else 2
+
+    def _strip_row0(self, hs: int, h: int) -> int:
+        """First image row of this rank's output strip (its patch)."""
+        if self.distri_config.n_device_per_batch == 1:
+            assert hs == h
+            return 0
+        return self.distri_config.split_idx() * hs
+
     def _step_kind(self) -> int:
         cfg = self.distri_config
         if self.counter <= cfg.warmup_steps or cfg.mode == "full_sync":
@@ -115,12 +128,7 @@ class DistriUNetPP(BaseModel):  # for Patch Parallelism
             if added_cond_kwargs is not None:
                 for k in added_cond_kwargs:
                     si["added_cond_kwargs"][k].copy_(added_cond_kwargs[k])
-            if self.counter <= cfg.warmup_steps:                     # distri_sdxl_unet_pp.py:108-113
-                graph_idx = 0
-            elif self.counter == cfg.warmup_steps + 1:
-                graph_idx = 1
-            else:
-                graph_idx = 2
+            graph_idx = self._graph_index()
             self.cuda_graphs[graph_idx].replay()
             if self.graph_launches is not None:
                 _lib.LAUNCHES["total"] += self.graph_launches[graph_idx]
@@ -139,15 +147,12 @@ class DistriUNetPP(BaseModel):  # for Patch Parallelism
                                 return_dict=False)[0]
             if cfg.world_size > 1 and live:                          # distri_sdxl_unet_pp.py:162-169 / 186-193
                 B = 2 if split else b
-                n = cfg.n_device_per_batch
                 if self.output_buffer is None:
                     self.output_buffer = torch.empty((B, c, h, w), device=output.device, dtype=output.dtype)
                 strip = output.contiguous()
                 bs, _, hs, _ = strip.shape
                 batch0 = cfg.batch_idx() if split else 0
-                row0 = cfg.split_idx() * hs if n > 1 else 0
-                if n == 1:
-                    assert hs == h
+                row0 = self._strip_row0(hs, h)
                 _lib.check(_lib.lib().df_output_gather(cm.world, strip.data_ptr(), self.output_buffer.data_ptr(), B, c, h, w,
                                                        bs, hs, batch0, row0, 0, cm.output_off,
                                                        torch.cuda.current_stream().cuda_stream), "df_output_gather")

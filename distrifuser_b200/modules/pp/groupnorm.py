@@ -18,13 +18,14 @@ class DistriGroupNorm(BaseModule):
     def __init__(self, module: nn.GroupNorm, distri_config: DistriConfig):
         assert isinstance(module, nn.GroupNorm)
         super().__init__(module, distri_config)
+        self.replicated = False         # set by tensor parallelism: every rank normalises its whole tensor, nothing is exchanged
         self.fuse_silu = False          # set by the block-level fusion in DistriUNetPP
         self._scratch = None
 
     def _plan(self):
         """-> (kernel mode, bessel, neg_var_fallback) for this call, following groupnorm.py:29-93."""
         cfg = self.distri_config
-        if cfg.n_device_per_batch == 1:
+        if cfg.n_device_per_batch == 1 or self.replicated:
             return MODE_LOCAL, 0, 0                                  # reference leaves the stock module (unwrapped)
         stat_modes = cfg.mode in ("stale_gn", "corrected_async_gn")
         neg_fb = int(cfg.mode == "corrected_async_gn")
@@ -50,7 +51,7 @@ class DistriGroupNorm(BaseModule):
         self._require_cuda_half(x, "DistriGroupNorm")
         b, c, h, w = x.shape
         G = module.num_groups
-        if cfg.n_device_per_batch > 1 and self._recording() and self.idx is None:
+        if cfg.n_device_per_batch > 1 and not self.replicated and self._recording() and self.idx is None:
             # the reference registers only in the two statistics modes (groupnorm.py:29-35); the peer-memory
             # exchange needs a slot in every mode that synchronises (sync_gn / full_sync / warm-up steps)
             self.idx = self.comm_manager.register_tensor([2, b, G, 1, 1, 1], torch.float32, layer_type="gn")

@@ -10,12 +10,15 @@ import os
 import torch
 
 from .models.distri_sdxl_unet_pp import DistriUNetPP
+from .models.distri_sdxl_unet_tp import DistriUNetTP
 from .utils import DistriConfig, PatchParallelismCommManager
 
 
 def _wrap(unet, distri_config: DistriConfig):
     if distri_config.parallelism == "patch":                         # pipelines.py:30-37
         return DistriUNetPP(unet, distri_config)
+    if distri_config.parallelism == "tensor":
+        return DistriUNetTP(unet, distri_config)
     raise ValueError(f"Unknown / unsupported parallelism: {distri_config.parallelism}")
 
 
@@ -74,7 +77,8 @@ class _DistriPipelineBase:
 
     @torch.no_grad()
     def _capture_graphs(self):
-        """Three graphs: synchronous step, first asynchronous step, steady state (pipelines.py:147-165)."""
+        """Three graphs: synchronous step, first asynchronous step, steady state (pipelines.py:147-165); tensor parallelism
+        has synchronous steps only and captures one (pipelines.py:154-155)."""
         cfg, unet, static_inputs = self.distri_config, self.pipeline.unet, self.static_inputs
         static_outputs, cuda_graphs = [], []
         unet.setup_cuda_graph(None, None, None)
@@ -82,7 +86,7 @@ class _DistriPipelineBase:
             if self.comm_manager is not None:
                 self.comm_manager.clear()
             torch.cuda.synchronize()
-            counters = [0, cfg.warmup_steps + 1, cfg.warmup_steps + 2]
+            counters = [0] if cfg.parallelism == "tensor" else [0, cfg.warmup_steps + 1, cfg.warmup_steps + 2]
             unet.static_inputs = None
             pool = None
             from . import _lib
@@ -91,7 +95,8 @@ class _DistriPipelineBase:
             # stream's 0): when a K/V projection finishes, the attention grid that follows it takes the SM slots before the
             # publication kernel of the same K/V does -- a publication CTA that got there first keeps a persistent attention
             # CTA out of its SM for the whole transfer (profiles/r2_exposed_comm_n8.txt)
-            prio = int(os.environ.get("DF_COMPUTE_PRIO", "-1" if cfg.n_device_per_batch > 1 else "0"))   # no publications without patch peers
+            patch_peers = cfg.n_device_per_batch > 1 and cfg.parallelism == "patch"
+            prio = int(os.environ.get("DF_COMPUTE_PRIO", "-1" if patch_peers else "0"))   # no publications without patch peers
             capture_stream = torch.cuda.Stream(device=cfg.device, priority=prio)
             for counter in counters:
                 graph = torch.cuda.CUDAGraph()

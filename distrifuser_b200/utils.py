@@ -15,7 +15,7 @@ import torch
 from torch import distributed as dist
 
 from . import _lib
-from ._lib import DfComm, NBANKS
+from ._lib import AR_RING, DfComm, NBANKS
 
 
 def is_power_of_2(n: int) -> bool:
@@ -54,10 +54,9 @@ class DistriConfig:
             f"distrifuser_b200 shards one image over the GPUs of ONE NVSwitch box (<= {_lib.MAX_WORLD} ranks, "
             f"DF_MAX_WORLD); got world_size={world_size}")
         assert mode in ("corrected_async_gn", "stale_gn", "sync_gn", "separate_gn", "full_sync", "no_sync")
-        if parallelism != "patch":
+        if parallelism not in ("patch", "tensor"):
             raise NotImplementedError(
-                "distrifuser_b200 implements the displaced patch-parallel path only (tensor / naive_patch are the "
-                "reference's comparison baselines and out of scope)")
+                f"parallelism={parallelism!r}: distrifuser_b200 implements \"patch\" and \"tensor\" (naive_patch is out of scope)")
 
         self.world_size = world_size
         self.rank = rank
@@ -80,6 +79,11 @@ class DistriConfig:
         else:
             n_device_per_batch = world_size
         self.n_device_per_batch = n_device_per_batch
+        if parallelism == "tensor" and n_device_per_batch == 1:
+            # the reference falls back to the unwrapped model here; this package has no second single-device path
+            raise NotImplementedError(
+                "parallelism=\"tensor\" over one device per CFG branch is the unsharded model: use parallelism=\"patch\", "
+                "which runs exactly that on one device")
 
         if torch.cuda.is_available():
             ndev = torch.cuda.device_count()
@@ -131,6 +135,11 @@ def _align(x: int, a: int) -> int:
     return (x + a - 1) // a * a
 
 
+def _dense(t: torch.Tensor) -> bool:
+    """[rows, C] in memory: NHWC (channels_last) for 4-D tensors, contiguous otherwise."""
+    return t.is_contiguous(memory_format=torch.channels_last) if t.ndim == 4 else t.is_contiguous()
+
+
 class _Holder:
     """Exposes a raw device allocation to torch through __cuda_array_interface__."""
 
@@ -158,6 +167,9 @@ class PatchParallelismCommManager:
         self.layer_types: list[str] = []
         self.output_spec = None          # (B, C, H, W) of the final epsilon, registered by DistriUNetPP
         self.output_off = 0
+        self.ar_bytes: list[int] = []    # payload bytes of every registered all-reduce site (tensor parallelism), in call order
+        self.ar_ring_off = 0
+        self.ar_slot_bytes = 0
         self.arena = None                # torch uint8 view of this rank's arena
         self._arena_ptr = None
         self._peer_ptrs: list[int] = []
@@ -192,16 +204,30 @@ class PatchParallelismCommManager:
     def register_output(self, B: int, Cc: int, H: int, W: int):
         self.output_spec = (B, Cc, H, W)
 
+    def register_allreduce(self, nbytes: int) -> int:
+        """One all-reduce site of the tensor-parallel path (called in execution order during the registration pass); returns
+        its site index.  The sites share one small ring of slots sized for the largest of them, so the arena does not grow
+        with their number."""
+        assert self.arena is None, "register_allreduce after create_buffer"
+        self.ar_bytes.append(int(nbytes))
+        return len(self.ar_bytes) - 1
+
     # ------------------------------------------------------------------ arena layout (pure host arithmetic)
     def _layout(self):
-        """Offsets of the symmetric arena: [group flags u32[nt][n] | world flags u32[world]] then DF_NBANKS banks, each
-        holding n source slots per registered tensor and one output image.  Returns (total_bytes, bank_stride)."""
+        """Offsets of the symmetric arena: [group flags u32[nt][n] | world flags u32[world] (| all-reduce flags
+        u32[DF_AR_RING][n])] then DF_NBANKS banks, each holding n source slots per registered tensor and one output image,
+        then (tensor parallelism) the all-reduce ring: DF_AR_RING x n slots of the largest registered all-reduce.
+        Returns (total_bytes, bank_stride)."""
         cfg = self.distri_config
         n, world = cfg.n_device_per_batch, cfg.world_size
         nt = len(self.slot_bytes)
         self._flags_group_off = 0
         self._flags_world_off = _align(4 * max(nt, 1) * n, 256)
         header = _align(self._flags_world_off + 4 * world, 1024)
+        self._flags_ar_off = 0
+        if self.ar_bytes:
+            self._flags_ar_off = _align(self._flags_world_off + 4 * world, 256)
+            header = _align(self._flags_ar_off + 4 * AR_RING * n, 1024)
         off = header
         self.tensor_off = []
         for sb in self.slot_bytes:
@@ -212,7 +238,10 @@ class PatchParallelismCommManager:
             B, Cc, H, W = self.output_spec
             off += _align(B * Cc * H * W * 2, 1024)
         bank_stride = _align(off - header, 1024)
-        return header + NBANKS * bank_stride, bank_stride
+        total = header + NBANKS * bank_stride
+        self.ar_slot_bytes = _align(max(self.ar_bytes), 256) if self.ar_bytes else 0
+        self.ar_ring_off = total
+        return total + AR_RING * n * self.ar_slot_bytes, bank_stride
 
     # ------------------------------------------------------------------ arena creation (utils.py:151-164)
     def create_buffer(self):
@@ -249,7 +278,7 @@ class PatchParallelismCommManager:
                 self._peer_ptrs.append(p.value)
         # local scratch: clock [4] u32, tickets [nt+1] u32
         self.clock = torch.zeros(4, dtype=torch.int32, device=cfg.device)
-        self._tickets = torch.zeros(nt + 2, dtype=torch.int32, device=cfg.device)
+        self._tickets = torch.zeros(nt + 3, dtype=torch.int32, device=cfg.device)   # [nt]: world gather, [nt + 2]: all-reduce
         members = cfg.patch_group_ranks()
         g = DfComm()
         for i, r in enumerate(members):
@@ -298,6 +327,17 @@ class PatchParallelismCommManager:
         return out
 
     # ------------------------------------------------------------------ step protocol
+    # ALL-REDUCE RING REUSE (tensor parallelism).  Every UNet call is a synchronous step (df_step_begin kind 0), and all-reduce
+    # `site` of the call with epoch e carries seq = e * nsites + site: consecutive all-reduces of a rank -- also across calls --
+    # have consecutive seq and alternate between the DF_AR_RING = 2 ring slots; flags are compared wrap-safely.  A rank that
+    # pushes all-reduce k+2 into slot (k % 2) of a peer has passed the wait of all-reduce k+1, i.e. seen that peer's k+1 flag;
+    # the peer stamps that flag in its k+1 kernel, which by stream order starts after its all-reduce k kernel -- the last read
+    # of slot (k % 2) -- completed.  So a slot is never overwritten while it is read, without any acknowledgement.  That holds
+    # only if an all-reduce kernel cannot start before the previous kernel of its stream has finished: df_allreduce_fwd is
+    # therefore always launched WITHOUT programmatic dependent launch, whatever DF_PDL selects for the other kernels (those
+    # touch no memory before griddepcontrol.wait, i.e. before the all-reduce that precedes them has completed).  Members
+    # that own no heads push nothing but still stamp and wait, so every member passes every all-reduce.
+    #
     # BANK-REUSE INVARIANT.  Bank e % 3 is overwritten by the peers' stores of epoch e+3 without any "consumed"
     # acknowledgement.  That is safe only because every UNet call ends with df_output_gather, which makes each rank wait
     # for the epsilon strip of EVERY world rank: no rank can start call t+1 before all ranks finished the kernels of call
@@ -309,6 +349,41 @@ class PatchParallelismCommManager:
         st = torch.cuda.current_stream().cuda_stream
         _lib.check(_lib.lib().df_step_begin(self.clock.data_ptr(), kind, st), "df_step_begin")
         self.epoch_host += 1
+
+    def all_reduce(self, site: int, partial: torch.Tensor | None, out: torch.Tensor, bias: torch.Tensor | None = None,
+                   residual: torch.Tensor | None = None, contrib_mask: int | None = None) -> torch.Tensor:
+        """out = sum of the patch group's partials + bias (+ residual) on every member (df_allreduce_fwd).  Tensors are NHWC
+        (channels_last) 4-D or [..., C] sequences, contiguous in that layout; partial None = this member owns nothing.  Before
+        create_buffer (registration pass) the result is this rank's partial + bias (+ residual): shapes only."""
+        cfg = self.distri_config
+        C = out.shape[1] if out.ndim == 4 else out.shape[-1]
+        rows = out.numel() // C
+        live = self.arena is not None
+        n = cfg.n_device_per_batch if live else 1
+        if contrib_mask is None:
+            contrib_mask = (1 << n) - 1
+        if not live:
+            comm, contrib_mask = _lib.null_comm(), int(partial is not None)
+        else:
+            comm = self.group
+        for t in (partial, residual):
+            assert t is None or (t.shape == out.shape and t.dtype == torch.float16 and _dense(t)), "all_reduce: layout"
+        assert _dense(out) and (bias is None or (bias.is_contiguous() and bias.numel() == C))
+        prof = _lib.PROFILE
+        if prof is not None:
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+        _lib.check(_lib.lib().df_allreduce_fwd(
+            comm, None if partial is None else partial.data_ptr(), out.data_ptr(), rows, C,
+            None if bias is None else bias.data_ptr(), None if residual is None else residual.data_ptr(), contrib_mask,
+            site, max(len(self.ar_bytes), 1), self.ar_ring_off, self.ar_slot_bytes, self._flags_ar_off if live else 0,
+            len(self.slot_bytes) + 2, torch.cuda.current_stream().cuda_stream), "df_allreduce_fwd")
+        if prof is not None:
+            e1.record()
+            nb = 2.0 * out.numel()
+            prof.append(dict(kernel="allreduce_kernel", kind="allreduce", flops=0.0, bytes=nb * (n + 2 + (residual is not None)),
+                             shape=(rows, C), start=e0, end=e1))
+        return out
 
     def group_mask(self) -> int:
         return (1 << self.distri_config.n_device_per_batch) - 1

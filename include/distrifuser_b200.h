@@ -35,6 +35,7 @@ extern "C" {
 #define DF_MAX_WORLD 8
 #define DF_IPC_HANDLE_BYTES 64
 #define DF_TENSORMAP_BYTES 128
+#define DF_AR_RING 2               /* depth of the all-reduce slot ring of the tensor-parallel path */
 
 /* ---- errors / info ------------------------------------------------------------------------------ */
 const char* df_last_error(void);
@@ -191,6 +192,22 @@ int df_linear_fwd(df_comm_t comm, const void* a, const void* w, const void* bias
                   int64_t M, int N, int K, int64_t lda, int64_t ldw, int64_t ldr, int64_t ldo, int epilogue,
                   int geglu_block, int publish, int pub_col0, int idx, uint32_t peer_mask, uint64_t tensor_off,
                   uint64_t slot_bytes, int max_ctas, void* stream);
+
+/* ---- tensor parallelism: fused all-reduce over peer memory.  Replaces the blocking dist.all_reduce + bias (+ residual)
+ *      adds of the reference's tensor-parallel modules (distrifuser/modules/tp/attention.py:159, feed_forward.py:77,
+ *      resnet.py:189, conv2d.py:52).
+ *      out[rows, C] = sum over members s in contrib_mask of partial_s + bias[C] (+ residual), fp32 in member order 0..n-1,
+ *      rounded to fp16 once: bit-identical on every member.  4-D NHWC tensors are passed as [b*h*w, C]; rows*C % 8 == 0.
+ *      partial == NULL: this member contributes nothing (it owns no heads); its bit in contrib_mask must then be clear.
+ *      One-shot: the partial goes to ring slot (seq % DF_AR_RING, src = comm.rank) of every peer, at arena offset
+ *      ring_off + (ring*world + src)*ring_slot_bytes, and the peer's flag u32 at flags_off + 4*(ring*world + src) is stamped
+ *      with seq = clock[0]*nsites + site (release, system scope); every member waits for all peers' flags (acquire) and
+ *      reduces locally.  After each df_step_begin the sites must be issued in order 0..nsites-1 on one stream, so that
+ *      consecutive all-reduces carry consecutive seq.  comm.tickets[ticket] is the CTA ticket.  comm.world == 1: no exchange.
+ *      Never launched with programmatic dependent launch (the ring reuse relies on stream order). ------------- */
+int df_allreduce_fwd(df_comm_t comm, const void* partial, void* out, int64_t rows, int C, const void* bias,
+                     const void* residual, uint32_t contrib_mask, int site, int nsites, uint64_t ring_off,
+                     uint64_t ring_slot_bytes, uint64_t flags_off, int ticket, void* stream);
 
 #ifdef __cplusplus
 }
